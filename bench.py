@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                  # this framework, BASELINE configs[1] per GPU
     python bench.py --impl reference --gpus N --steps K ...        # the reference's own CPU path on the host cores
     python bench.py --workload cfg4|render|sweep ...               # the other BASELINE configs (see below)
+    python bench.py --steps K --warmup W --dump-outputs DIR        # + the last timed step's outputs as DIR/<name>.npy
 
 Default workload (BASELINE.json configs[1]): one training step of configs/example_sequence.txt -- N_rand = 1024 rays per
 GPU, 64 coarse + 128 fine network evaluations per ray, 8x256 MLP, ray bending on, perturb = 1, raw_noise_std = 1,
@@ -229,7 +230,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="run the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--no-breakdown", action="store_true", help="skip the instrumented per-kernel pass")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (mean and per-ray loss, updated parameters, their gradients) "
+                         "as DIR/<name>.npy, to compare two builds on identical inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload in ("render", "sweep")):
+        ap.error("--dump-outputs applies to this implementation's training step (--workload train or cfg4)")
     args.warmup = max(args.warmup, 3)
     if args.n_rand is None:
         args.n_rand = 8192 if args.workload == "cfg4" else N_RAND
@@ -313,7 +321,7 @@ def main():
             optimizer.step()                                     # 1 GPU: Adam; N GPUs: peer reduce + Adam, same launch
             gathered = peer_red.gather_rows(losses) if peer_red is not None else losses.detach()
             global_step.add_(1.0)
-            return gathered.mean()
+            return gathered.mean(), gathered
         return losses.detach()
 
     graphed = None
@@ -341,7 +349,7 @@ def main():
         global_step.add_(1.0)
         gathered = torch.empty(world * (hi - lo), dtype=out.dtype, device=dev)
         dist.all_gather_into_tensor(gathered, out.contiguous())
-        return gathered.mean()
+        return gathered.mean(), gathered
 
     def barrier():
         if world > 1:
@@ -355,24 +363,31 @@ def main():
         for i in range(loop_steps):
             if e2e:
                 # host -> device copy of this step's inputs from pinned memory (straight into the graph's input buffers)
-                loss = step(pinned[i % pool] if graphed is not None else upload(pinned[i % pool]))
-                loss.item()                              # device -> host read of the step's result
+                out = step(pinned[i % pool] if graphed is not None else upload(pinned[i % pool]))
+                out[0].item()                            # device -> host read of the step's result
             else:
-                step(resident[i % pool])
+                out = step(resident[i % pool])
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), out
 
     for i in range(args.warmup):
         step(resident[i % pool])
     _lib.device_error_check()
 
     sampler = ClockSampler(local_rank) if rank == 0 else None
-    ms_total = timed(args.steps, e2e=False)      # headline: the plain step (no instrumentation inside the graph)
-    ms_e2e = timed(args.steps, e2e=True)
+    ms_total, last = timed(args.steps, e2e=False)      # headline: the plain step (no instrumentation inside the graph)
+    # copied to the host at once: the graph's output buffers are overwritten by the windows that follow
+    outputs = None
+    if args.dump_outputs and rank == 0:
+        outputs = {"loss": last[0], "ray_loss": last[1],
+                   "params": torch.cat([p.detach().reshape(-1) for p in grad_vars]),
+                   "grads": torch.cat([p.grad.reshape(-1) for p in grad_vars])}
+        outputs = {k: v.float().cpu().numpy() for k, v in outputs.items()}
+    ms_e2e, _ = timed(args.steps, e2e=True)
     clocks = sampler.stop() if sampler else None
     # per-kernel breakdown: the same K steps once more with CUDA event records around every launch of this repo's
     # kernels (external event-record nodes inside the re-captured graph; they cost a few us per step themselves)
@@ -386,7 +401,7 @@ def main():
             graphed = GraphedStep(local_step, resident[0], warmup=1)
             for i in range(3):
                 step(resident[i % pool])
-        ms_instrumented = timed(args.steps, e2e=False)
+        ms_instrumented, _ = timed(args.steps, e2e=False)
         kinds = _lib.timing_read()
         _lib.timing_enable(False)
         # launches per step: forward / DGRAD / composite / composite backward 2 (coarse + fine), divergence 2 (fwd + bwd),
@@ -395,7 +410,7 @@ def main():
         per_step = {k: (kinds[k][0] / (kinds[k][1] / float(launches.get(k, 2))) if kinds[k][1] else 0.0) for k in kinds}
     _lib.device_error_check()
 
-    final_loss = float(step(resident[0]).item())
+    final_loss = float(step(resident[0])[0].item())
     if peer_red is not None:
         peer_red.close()
     if world > 1:
@@ -403,6 +418,11 @@ def main():
         dist.destroy_process_group()
     if rank != 0:
         return
+    if outputs is not None:
+        # float32; about 9 MB in all (1.07 M parameters and as many gradients, one loss per ray of the global batch)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
 
     value = n_global * args.steps / (ms_total * 1e-3)
     e2e_value = n_global * args.steps / (ms_e2e * 1e-3)

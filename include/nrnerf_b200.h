@@ -299,7 +299,8 @@ int nrn_peer_gather_rows(const NrnPeerCtx* ctx, const float* local, int n_per_ra
 /* ---- optional per-kernel timing (measurement aid for bench.py) ---------------------------------
  * While enabled, every launch of the kernel kinds below is bracketed by CUDA events recorded on the
  * launch stream.  kinds: 0 field forward, 1 field DGRAD, 2 WGRAD (+reduce), 3 composite(+resample),
- * 4 composite backward, 5 divergence regulariser.  nrn_timing_read synchronises the recorded events and returns per-kind sums. */
+ * 4 composite backward, 5 divergence regulariser.  nrn_timing_read synchronises the recorded events and returns per-kind sums.
+ * The events live until the process ends, so a graph captured while timing was on may be replayed after it is turned off. */
 int nrn_timing_enable(int on);
 int nrn_timing_read(double* ms_sum, int* counts, int n_kinds);
 

@@ -79,7 +79,7 @@ struct ScopedTimer {
   ScopedTimer(int kind, cudaStream_t s) : st(s) {
     if (!g_timing || g_timed_n >= 4096) return;
     TimedLaunch& t = g_timed[g_timed_n];
-    if (cudaEventCreate(&t.a) != cudaSuccess || cudaEventCreate(&t.b) != cudaSuccess) return;
+    if ((!t.a && cudaEventCreate(&t.a) != cudaSuccess) || (!t.b && cudaEventCreate(&t.b) != cudaSuccess)) return;
     t.kind = kind;
     idx = g_timed_n++;
     record(t.a);
@@ -572,7 +572,8 @@ int nrn_peer_gather_rows(const NrnPeerCtx* c, const float* local, int n_per_rank
 }
 
 int nrn_timing_enable(int on) {
-  for (int i = 0; i < g_timed_n; ++i) { cudaEventDestroy(g_timed[i].a); cudaEventDestroy(g_timed[i].b); }
+  // the events are reused, never destroyed: a graph captured while timing was on holds event-record nodes naming them,
+  // and replaying it after they were destroyed makes cudaGraphLaunch read freed memory
   g_timed_n = 0;
   g_timing = on != 0;
   return NRN_OK;
